@@ -15,11 +15,19 @@ forward+loss+backward of `n` of the 28 blocks at full width, `n` sized so the K+
 `ms_per_step` is the time of that sample and `value` the tokens/s it extrapolates to (x 28/n), both stated in the line.
 `--impl reference-gpu` (informational, not part of the driver contract): the same oracle moved to cuda:0 in bf16 with
 PyTorch SDPA and per-block activation checkpointing - the "PyTorch eager on the same box" bar of SURVEY section 0.
+`--dump-outputs DIR` (b200 arm, rank 0) writes what the last of the K steps timed for `value` handed its caller as
+DIR/<name>.npy in float32 (see step_outputs).  Model, data, sigmas, noise and first-frame draws are all seeded, so two
+builds run with the same arguments see the same inputs and can be compared output for output.  Outputs are not bitwise
+reproducible: the attention backward and the LoRA weight-gradient GEMMs accumulate with fp32 atomics in a varying order,
+and the drift compounds over the steps.  Two runs of one build (`--steps 10 --warmup 3`, one NVIDIA B200 at its 1000 W
+power limit) agreed, as max |difference| / max |value|, to 2e-6 in loss, 5e-5 in grad_norm, 3e-6 in lora_weights, 5e-4
+in lora_exp_avg and 1.1e-2 in the bf16 prediction.
 """
 import argparse
 import json
 import math
 import os
+import random
 import statistics
 import sys
 import threading
@@ -36,6 +44,7 @@ TEXT_LEN = 128
 RANK_LORA = 64
 N_BLOCKS = 28
 FLOP_PER_TOKEN_ALG = 8.88e9              # SURVEY §8(d): 2G + 3.5A, no recompute counted
+DUMP_SAMPLE = 1 << 20                    # --dump-outputs: larger outputs keep a fixed, seeded sample of this many elements
 
 
 def workload_config(B, world, parallelism="ddp"):
@@ -253,6 +262,24 @@ def run_reference_gpu(args):
 # ----------------------------------------------------------------------------------------------------------------------
 # b200 arm
 # ----------------------------------------------------------------------------------------------------------------------
+def step_outputs(step, model, B):
+    """What the last optimizer step left its caller, as float32 host arrays: the step's loss and gradient norm, the model's
+    prediction for the batch [B, 2688, 128], the updated flat fp32 LoRA weights and AdamW's first moment.  The moment
+    stands in for the gradient, which the fused AdamW kernel zeroes.  An output of more than DUMP_SAMPLE elements (the
+    two flat buffers: ~59M each) keeps the same seeded sample of positions in every run."""
+    import torch
+    outs = {"loss": step.metrics[1:2], "grad_norm": step.metrics[0:1],
+            "pred": model._workspace(B, S_TOK, TEXT_LEN)["pred"].view(B, S_TOK, -1),
+            "lora_weights": model.lora_flat, "lora_exp_avg": step.exp_avg}
+    host = {}
+    for name, t in outs.items():
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        host[name] = t.float().cpu().numpy()
+    return host
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -280,6 +307,7 @@ def run_b200(args):
 
     # ---- model: LTX-2B architecture, random init (no checkpoints offline), LoRA r=64 on to_q|to_k|to_v|to_out.0
     torch.manual_seed(0)
+    random.seed(0)                    # the first-frame-conditioning draw of every micro-step (random.random())
     model = B200LTXTransformer(LTXConfig(), torch.bfloat16, dev)
     with torch.no_grad():
         for n, p in model.named_parameters():
@@ -371,6 +399,8 @@ def run_b200(args):
         step_resident(i)
     mark0 = sampler.mark() if sampler else 0
     ms_total, per_step = timed(step_resident, args.steps)
+    # taken here, not after a re-measurement below: what is dumped must not depend on how noisy the timing was
+    dumped = step_outputs(step, model, B) if (args.dump_outputs and rank == 0) else None
     for i in range(2):
         step_e2e(i)
     ms_e2e, per_e2e = timed(step_e2e, args.steps)
@@ -479,6 +509,11 @@ def run_b200(args):
         line["fsdp"] = {"local_param_bytes": fs.local_param_bytes(), "full_bytes_per_block": fs.full_bytes_per_block,
                         "allgathers_per_step": (2 * (fs.nl - 2) + 1), "note": "per-block bf16 all-gather prefetched one block "
                         "ahead on a communication stream; fp32 reduce-scatter of the flat LoRA gradient; sharded AdamW"}
+    if dumped is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
     print(json.dumps(line))
     if be is not None:
         be.destroy()
@@ -496,7 +531,13 @@ def main():
     ap.add_argument("--ddp-chunks", type=int, default=4, help="N > 1, ddp: block-range chunks of the overlapped gradient exchange (1 = one serial all-reduce)")
     ap.add_argument("--parallelism", default="ddp", choices=["ddp", "fsdp"],
                     help="N > 1: ddp = replicas + flat gradient all-reduce (default); fsdp = FSDP-2 per-block sharding")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32; b200 arm only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs is only implemented for --impl b200")
     if args.impl == "reference":
         run_reference(args)
     elif args.impl == "reference-gpu":
